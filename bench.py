@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- FAcodec encode -> quantize -> decode throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (encoder -> quantizer(n_c=2, codes) -> decoder) over one
 batch of synthetic 4 s 24 kHz utterances (PseudoDataset law, meldataset.py:67-68); the workload
@@ -15,8 +15,10 @@ Prints ONE JSON line on rank 0 (contract in the task statement):
                ncu launch list (profiles/roofline_r02.json)
   cpu_baseline = the oracle port (oracle/facodec_oracle.py = the reference's own ATen call sequence)
                timed on this box's host cores on a bounded sample
---impl reference times that CPU path alone (the reference is 100% Python/PyTorch; /root/reference is
-not on the GPU box, so the validated restatement stands in: kind "port").
+--impl reference times that CPU path alone (the reference is 100% Python/PyTorch, so the validated restatement
+stands in: kind "port").
+--dump-outputs DIR writes what the last timed step returned (waveforms, the three code tensors, timbre vectors of rank 0)
+as DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -94,6 +96,21 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(out_dir, arrays, limit_bytes=64 << 20):
+    """Writes each tensor as out_dir/<name>.npy: float32, or float64 for integer tensors (code indices stay exact)."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a.astype(np.float64 if a.dtype.kind in "iub" else np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > limit_bytes:
+        raise ValueError(f"outputs take {total} bytes, more than the {limit_bytes} a dump may hold")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def usable_cores():
@@ -321,7 +338,13 @@ def main():
     ap.add_argument("--workload", default="codec", choices=["codec", "vq", "trainfwd"],
                     help="codec = BASELINE configs[1] (the headline); vq = configs[3] FVQ/RVQ codebook-distance microbench; "
                          "trainfwd = the forward half of configs[4] (codec forward + losses.reconstruction_loss)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (codec workload, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "codec" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the codec workload's timed path (--workload codec --impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -410,8 +433,20 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(lambda i: codec.forward(xs[i % nrot], n_c=2), args.steps)
+    last = []
+
+    def step(i):
+        out = codec.forward(xs[i % nrot], n_c=2)
+        if i == args.steps - 1:
+            last.append(out)
+
+    ms_total = timed(step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        y_last, codes_last, timbre_last = last[0]
+        dump_outputs(args.dump_outputs, {"y": y_last, "codes_p": codes_last[0], "codes_c": codes_last[1],
+                                         "codes_r": codes_last[2], "timbre": timbre_last})
+    del last
     launches = codec.launch_count() * args.steps
     audio_s = world * BATCH_PER_GPU * UTT_SECONDS * args.steps
     value = audio_s / (ms_total * 1e-3)

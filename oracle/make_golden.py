@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.npz by running the
-*unmodified imported reference* (oracle/ref_import.py) on CPU, in the build
-container (needs /root/reference).  Run:  python -m oracle.make_golden
+*unmodified imported reference* (oracle/ref_import.py) on CPU; needs a checkout
+of the reference at ref_import.REFERENCE_ROOT.
+Run:  python -m oracle.make_golden [pins | recon_loss | redecoder]
 
 Weights come from facodec_b200.synth.synth_state_dicts(seed) (host-independent
 bits) loaded into the reference modules with load_state_dict, exactly as
@@ -144,8 +145,199 @@ def main_recon_loss():
     print("recon_loss", float(loss), [float(t) for t in terms])
 
 
+# ---------------------------------------------------------------------------------------------------------------
+# Pins of the restatement: what the imported reference modules return for the inputs of tests/test_oracle.py, stored
+# under tests/golden/pin_*, so that those tests compare against the reference on any box.
+# ---------------------------------------------------------------------------------------------------------------
+SAMPLE_N = 2048
+
+
+def sample(a, n=SAMPLE_N):
+    """A fixed, seeded subset of the (flattened) elements of a large array; arrays of at most n elements stay whole."""
+    flat = np.asarray(a).reshape(-1)
+    if flat.size <= n:
+        return flat
+    return flat[np.sort(np.random.RandomState(0).choice(flat.size, n, replace=False))]
+
+
+def pinned(**arrays):
+    """name -> sample(array) plus name + '_shape' -> its full shape."""
+    out = {}
+    for k, v in arrays.items():
+        v = v.detach().numpy() if torch.is_tensor(v) else np.asarray(v)
+        out[k] = sample(v)
+        out[k + "_shape"] = np.array(v.shape, np.int64)
+    return out
+
+
+def seeded_tensors(names, shapes, seed):
+    """Host-independent stand-in weights: N(0, 1 / fan_in) per tensor, drawn in the order given."""
+    g = torch.Generator().manual_seed(seed)
+    out = {}
+    for k, s in zip(names, shapes):
+        s = tuple(int(d) for d in s)
+        fan_in = int(np.prod(s[1:])) if len(s) > 1 else 1
+        out[k] = torch.randn(s, generator=g) / float(np.sqrt(fan_in))
+    return out
+
+
+def shape_strings(tensors):
+    return np.array([",".join(str(d) for d in t.shape) for t in tensors])
+
+
+def parse_shapes(strings):
+    return [tuple(int(d) for d in s.split(",") if d) for s in strings]
+
+
+PIN_CODEC = dict(wseed=1, xseed=21, B=2, T=4500, n_c=2)
+PIN_RVQ = dict(num_quantizers=4, codebook_size=10, dim=1024, codebook_dim=8, commitment=0.25, wseed=3, xseed=3, T=17)
+PIN_RECON_LOSS = dict(B=3, T=7000, seed=5)
+PIN_FAP_FLAGS = dict(use_gr_content_f0=False, use_gr_prosody_phone=False, use_gr_residual_f0=True, use_gr_residual_phone=True,
+                     use_gr_timbre_content=True, use_gr_timbre_prosody=False, use_gr_x_timbre=True, norm_f0=True)   # modules/commons.py:311-322 + config.yml
+
+
+def pin_path(name):
+    return os.path.join(GOLDEN_DIR, name)
+
+
+def main_pins():
+    import warnings
+    warnings.simplefilter("ignore")
+    ref_import.import_reference()
+    saved = {}
+
+    # codec: encoder -> quantizer -> decoder of build_model(config.yml) with synthetic weights
+    c = PIN_CODEC
+    model = ref_import.build_reference_model(0)
+    sds = synth.synth_state_dicts(c["wseed"])
+    for k in ("encoder", "quantizer", "decoder"):
+        model[k].load_state_dict(sds[k])
+    x = synth.synth_waves(c["B"], c["T"], seed=c["xseed"])
+    with torch.no_grad():
+        z = model.encoder(x)
+        q = model.quantizer(z, x, n_c=c["n_c"], return_codes=True)
+        y = model.decoder(q[0])
+    saved["pin_codec.npz"] = dict(pinned(z=z, outs=q[0], timbre=q[4], y=y, z_p=q[1][0], z_c=q[1][1], z_r=q[1][2]),
+                                  codes_p=q[5][0].numpy(), codes_c=q[5][1].numpy(), codes_r=q[5][2].numpy(),
+                                  commitment=q[2].numpy(), codebook=q[3].numpy())
+
+    # quantize/rvq.py ResidualVQ with seeded weights, and alias_free_torch.Activation1d(Identity)
+    from quantize.rvq import ResidualVQ as RefRVQ
+    from alias_free_torch import Activation1d as RefAct
+    r = PIN_RVQ
+    rvq = RefRVQ(num_quantizers=r["num_quantizers"], codebook_size=r["codebook_size"], dim=r["dim"],
+                 codebook_dim=r["codebook_dim"], commitment=r["commitment"]).eval()
+    names = list(rvq.state_dict())
+    shapes = shape_strings(rvq.state_dict().values())
+    rvq.load_state_dict(seeded_tensors(names, parse_shapes(shapes), r["wseed"]))
+    g = torch.Generator().manual_seed(r["xseed"])
+    x = torch.randn(2, r["dim"], r["T"], generator=g)
+    xx = torch.randn(2, 5, 50, generator=g)
+    with torch.no_grad():
+        a = rvq(x)
+        act = RefAct(activation=torch.nn.Identity())(xx)
+    saved["pin_rvq_altfree.npz"] = dict(pinned(quantized=a[0], act=act), names=np.array(names), shapes=shapes,
+                                        indices=a[1].numpy(), all_quantized=sample(a[3].numpy()))
+
+    # modules/redecoder.py encoder + the non-causal, LSTM-free decoder of build_model(stage='redecoder')
+    model = ref_import.build_reference_redecoder(0)
+    sds = synth.synth_redecoder_state_dicts(2)
+    for k in ("encoder", "decoder"):
+        model[k].load_state_dict(sds[k])
+    g = torch.Generator().manual_seed(5)
+    cp = torch.randint(0, 1024, (2, 1, 13), generator=g)
+    cc = torch.randint(0, 1024, (2, 2, 13), generator=g)
+    timbre = torch.randn(2, 1024, generator=g)
+    out = {}
+    for use_p, n_c in ((False, 1), (True, 2)):
+        with torch.no_grad():
+            z = model.encoder(cp, cc, timbre, use_p_code=use_p, n_c=n_c)
+            y = model.decoder(z)
+        out.update(pinned(**{f"z_{int(use_p)}{n_c}": z, f"y_{int(use_p)}{n_c}": y}))
+    saved["pin_redecoder.npz"] = out
+
+    # SnakeBeta inside Activation1d, CNNLSTM heads (modules/quantize.py)
+    from modules.quantize import CNNLSTM, SnakeBeta
+    g = torch.Generator().manual_seed(9)
+    sb = SnakeBeta(6, alpha_logscale=True)
+    with torch.no_grad():
+        sb.alpha.copy_(torch.randn(6, generator=g) * 0.3)
+        sb.beta.copy_(torch.randn(6, generator=g) * 0.3)
+    x = torch.randn(2, 6, 40, generator=g)
+    with torch.no_grad():
+        out = dict(snake=sb(x).numpy(), snake_act=RefAct(activation=sb)(x).numpy())
+    for i, (indim, outdim, heads, glob) in enumerate(((64, 10, 2, False), (32, 7, 1, True))):
+        m = CNNLSTM(indim, outdim, heads, global_pred=glob).eval()
+        m.load_state_dict(synth.synth_cnnlstm(3, indim, outdim, heads), strict=False)
+        out[f"keys_{i}"] = np.array(list(m.state_dict()))
+        xx = torch.randn(2, indim, 33, generator=g)
+        with torch.no_grad():
+            for h, t in enumerate(m(xx)):
+                out[f"head_{i}_{h}"] = t.numpy()
+    saved["pin_heads.npz"] = out
+
+    # meldataset.py preprocess (torchaudio MelSpectrogram): output, window and (sparse) filterbank it used
+    import meldataset
+    w = synth.synth_waves(1, 5000, seed=3)[0, 0]
+    with torch.no_grad():
+        ref = meldataset.preprocess(w.numpy())
+    fb = meldataset.to_mel.mel_scale.fb
+    nz = torch.nonzero(fb.reshape(-1)).reshape(-1)
+    saved["pin_dataset_mel.npz"] = dict(mel=ref.numpy(), window=meldataset.to_mel.spectrogram.window.numpy(),
+                                        fb_shape=np.array(fb.shape, np.int64), fb_index=nz.numpy().astype(np.int32),
+                                        fb_value=fb.reshape(-1)[nz].numpy())
+
+    # losses.py reconstruction_loss
+    import losses as ref_losses
+    c = PIN_RECON_LOSS
+    x, G_x = synth.synth_loss_pair(c["B"], c["T"], c["seed"])
+    with torch.no_grad():
+        saved["pin_recon_loss.npz"] = dict(loss=ref_losses.reconstruction_loss(x, G_x).numpy(), **c)
+
+    # FApredictors (modules/quantize.py) with build_model's flags, seeded parameters, both forward variants
+    from modules.quantize import FApredictors
+    out = {}
+    for tn in (True, False):
+        m = FApredictors(in_dim=32, timbre_norm=tn, use_gr_content_global_f0=True, **PIN_FAP_FLAGS).eval()
+        params = dict(m.named_parameters())
+        names = list(params)
+        shapes = shape_strings(params.values())
+        missing, unexpected = m.load_state_dict(seeded_tensors(names, parse_shapes(shapes), 4), strict=False)
+        assert not unexpected
+        bufs = {k: v for k, v in m.state_dict().items() if k not in params}
+        assert sorted(missing) == sorted(bufs)
+        g = torch.Generator().manual_seed(6)
+        lat = [torch.randn(2, 32, 19, generator=g) for _ in range(3 if tn else 4)]
+        with torch.no_grad():
+            res = m(lat, torch.randn(2, 32, generator=g)) if tn else m(lat)
+        p = f"tn{int(tn)}_"
+        out[p + "names"] = np.array(names)
+        out[p + "shapes"] = shapes
+        out[p + "buffer_names"] = np.array(list(bufs))
+        out[p + "buffer_shapes"] = shape_strings(bufs.values())
+        out[p + "buffers"] = torch.cat([b.reshape(-1) for b in bufs.values()]).numpy()
+        out.update(pinned(**{p + k: v for d in res for k, v in d.items() if v is not None}))
+        out[p + "none"] = np.array([k for d in res for k, v in d.items() if v is None])
+    saved["pin_fa_predictors.npz"] = out
+
+    for name, arrays in saved.items():
+        np.savez_compressed(pin_path(name), **arrays)
+        print(name, os.path.getsize(pin_path(name)) // 1024, "KiB")
+
+    # dac/model/base.py DACFile: the bytes its save() writes
+    from dac.model.base import DACFile as RefFile
+    from facodec_b200 import codefile
+    g = torch.Generator().manual_seed(9)
+    codes = [torch.randint(0, 1024, (2, n, 37), generator=g) for n in (1, 2, 3)]
+    ref = RefFile(codes=codefile.pack_codes(codes), chunk_length=37, original_length=37 * 300,
+                  input_db=torch.tensor([-23.5, -17.25]), channels=1, sample_rate=24000, padding=True, dac_version="1.0.0")
+    print(ref.save(pin_path("pin_codefile.dac")))
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "recon_loss":
+    if len(sys.argv) > 1 and sys.argv[1] == "pins":
+        main_pins()
+    elif len(sys.argv) > 1 and sys.argv[1] == "recon_loss":
         main_recon_loss()
     elif len(sys.argv) > 1 and sys.argv[1] == "redecoder":
         main_redecoder()
