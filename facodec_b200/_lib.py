@@ -45,6 +45,8 @@ def load():
         "fac_redecode": ([vp, i64p, i64p, i32, fp, i32, i32, i32, i32, i32, fp, vp], i32),
         "fac_redecoder_decode": ([vp, fp, i32, i32, fp, vp], i32),
         "fac_voice_convert": ([vp, i64p, i64p, i32, fp, i32, i32, i32, i32, i32, fp, vp], i32),
+        "fac_dequantize": ([vp, i64p, i64p, i32, i32, i64p, i32, i32, fp, i32, i32, fp, fp, fp, fp, vp], i32),
+        "fac_decode_codes": ([vp, i64p, i64p, i32, i32, i64p, i32, i32, fp, i32, i32, fp, vp], i32),
         "fac_dataset_mel": ([vp, fp, i32, i32, fp, vp], i32),
         "fac_head_begin": ([vp], i32),
         "fac_head_tensor": ([vp, i32, _c.c_char_p, fp, _c.POINTER(_c.c_int64), i32], i32),
@@ -96,7 +98,7 @@ def load():
 
 EXPORTED = ["fac_abi_version", "fac_create", "fac_destroy", "fac_last_error", "fac_load_tensor", "fac_finalize",
             "fac_encode", "fac_encode_frames", "fac_quantize", "fac_decode", "fac_codec_forward",
-            "fac_codec_forward_host", "fac_redecode", "fac_redecoder_decode", "fac_voice_convert", "fac_dataset_mel", "fac_reconstruction_loss", "fac_spectral_loss", "fac_l1_loss", "fac_head_begin", "fac_head_tensor", "fac_head_finalize", "fac_head_forward", "fac_add3", "fac_stream_begin", "fac_stream_encode", "fac_stream_decode", "fac_stream_end", "fac_rvq_create", "fac_rvq_destroy", "fac_rvq_forward", "fac_alias_free_act",
+            "fac_codec_forward_host", "fac_redecode", "fac_redecoder_decode", "fac_voice_convert", "fac_dequantize", "fac_decode_codes", "fac_dataset_mel", "fac_reconstruction_loss", "fac_spectral_loss", "fac_l1_loss", "fac_head_begin", "fac_head_tensor", "fac_head_finalize", "fac_head_forward", "fac_add3", "fac_stream_begin", "fac_stream_encode", "fac_stream_decode", "fac_stream_end", "fac_rvq_create", "fac_rvq_destroy", "fac_rvq_forward", "fac_alias_free_act",
             "fac_debug_conv", "fac_debug_conv_tc", "fac_debug_resunit", "fac_debug_tc_phase_clocks", "fac_debug_tc_producer_clocks", "fac_debug_tc_trace", "fac_debug_lstm_pack", "fac_debug_convtr_pack", "fac_debug_pad_map", "fac_debug_tc_plan", "fac_debug_tc_pack", "fac_debug_lstm_phase_clocks", "fac_set_option", "fac_debug_slstm", "fac_debug_tap", "fac_profile_enable", "fac_profile_reset", "fac_profile_get", "fac_profile_dump",
             "fac_workspace_bytes", "fac_last_launch_count"]
 

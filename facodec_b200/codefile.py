@@ -81,3 +81,14 @@ def from_forward(codes: Sequence[torch.Tensor], original_length: int, sample_rat
     return DACFile(codes=packed, chunk_length=packed.shape[-1] if chunk_length is None else chunk_length,
                    original_length=int(original_length), input_db=input_db, channels=channels, sample_rate=sample_rate,
                    padding=padding, dac_version=SUPPORTED_VERSIONS[-1])
+
+
+def decode(model, dac_or_path, timbre, n_c: int = 2, n_r: int = None) -> torch.Tensor:
+    """Audio from a ``.dac`` file (a path or a loaded :class:`DACFile`) of a build_model() Munch: unpack the codes (``n_c``
+    content rows per the file's layout), move them to ``timbre``'s device and run ``Codec(model).decode_codes``.  The
+    format holds codes only, so the timbre [B, 1024] (one vector per utterance, e.g. the forward's own) is an argument;
+    ``n_r`` residual codebooks are used (default: all in the file).  Returns y [B, 1, 300 T']."""
+    from .modules import Codec
+    f = dac_or_path if isinstance(dac_or_path, DACFile) else DACFile.load(dac_or_path)
+    codes = [c.to(timbre.device) for c in unpack_codes(f.codes, n_c=n_c)]
+    return Codec(model).decode_codes(codes, timbre, n_c=n_c, n_r=n_r)

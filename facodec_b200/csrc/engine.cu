@@ -1204,6 +1204,40 @@ void join_front(Ctx& c) {
     if (!c.dry) c.check_nk(cudaStreamWaitEvent(c.st, c.h->ev_join, 0), "front.join_wait");
 }
 
+// Decoding from codes: ResidualVectorQuantize.from_codes of each group (dac/nn/quantize.py:200-220) and the forward_v2
+// tail (modules/quantize.py:435-449).  gamma, beta = timbre_linear(timbre) in the precision class quantizer_front uses,
+// so the forward's own timbre gives the forward's gamma_beta bit for bit; then one dequantize_kernel.  Returns
+// channels-last outs [B][T][1024] in workspace; zp_cl / zc_cl / zr_cl (channels-last, may be null) receive the groups.
+float* dequantize_forward(Ctx& c, const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, int n_c, const int64_t* codes_r,
+                          int n_r_rows, int n_r, const float* timbre, int B, int T, float* zp_cl, float* zc_cl, float* zr_cl) {
+    const QuantW& q = c.h->qw;
+    float* gb = c.alloc<float>((size_t)B * 2048);
+    float* outs = c.alloc<float>((size_t)B * T * LATENT);
+    const bool was_critical = c.vq_critical;
+    c.vq_critical = true;
+    run_conv(c, q.timbre_linear, timbre, gb, 1, B, B, ConvOpts(), "timbre_linear");
+    c.vq_critical = was_critical;
+    c.tap("gamma_beta", gb, (size_t)B * 2048);
+    if (c.dry) return outs;
+    DequantParams dp;
+    dp.codes_p = codes_p; dp.codes_c = codes_c; dp.codes_r = codes_r;
+    dp.n_c_rows = n_c_rows; dp.n_c = n_c; dp.n_r_rows = n_r_rows; dp.n_r = n_r;
+    for (int i = 0; i < 6; ++i) {
+        const VqW& v = q.vq[i];
+        dp.vq[i] = VqWeights{c.W(v.w_in), c.W(v.b_in), c.W(v.cb), c.W(v.cbn), c.W(v.cbn2), c.W(v.w_out), c.W(v.b_out)};
+    }
+    dp.gamma_beta = gb;
+    dp.outs = outs; dp.zp = zp_cl; dp.zc = zc_cl; dp.zr = zr_cl;
+    dp.B = B; dp.T = T;
+    const double frames = (double)B * T;
+    const int parts = (zp_cl ? 1 : 0) + (zc_cl ? 1 : 0) + (zr_cl ? 1 : 0);
+    c.begin("dequantize", 2.0 * frames * (1 + n_c + n_r) * 8.0 * LATENT,   // 8 = codebook dim
+            4.0 * frames * LATENT * (1 + parts) + 8.0 * frames * (1 + n_c + n_r));
+    c.check(launch_dequantize(dp, c.st), "dequantize");
+    c.end();
+    return outs;
+}
+
 int ensure_ws(fac_handle* h, size_t bytes) {
     if (bytes <= h->ws_bytes) return FAC_OK;
     if (h->ws) { cudaDeviceSynchronize(); cudaFree(h->ws); h->ws = nullptr; h->ws_bytes = 0; }
@@ -1468,6 +1502,50 @@ int fac_voice_convert(fac_handle* h, const int64_t* codes_p, const int64_t* code
     return two_pass(h, (cudaStream_t)stream, [&](Ctx& c) {
         float* zcl = redecoder_forward(c, codes_p, codes_c, n_c_rows, timbre, B, T, use_p_code, use_c_code, n_c);
         decoder_forward(c, h->dec2, zcl, B, T, y);
+    });
+}
+
+static bool dequant_args_ok(const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, int n_c, const int64_t* codes_r,
+                            int n_r_rows, int n_r, const float* timbre, int B, int T) {
+    return codes_p && codes_c && timbre && B > 0 && T > 0 && n_c >= 1 && n_c <= n_c_rows && n_c_rows <= 2 && n_r >= 0 &&
+           n_r <= n_r_rows && n_r_rows <= 3 && (n_r == 0 || codes_r);
+}
+
+int fac_dequantize(fac_handle* h, const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, int n_c, const int64_t* codes_r,
+                   int n_r_rows, int n_r, const float* timbre, int B, int T, float* outs, float* zp, float* zc, float* zr,
+                   void* stream) {
+    int rc = check_ready(h, FAC_QUANTIZER);
+    if (rc) return rc;
+    if (!outs || !dequant_args_ok(codes_p, codes_c, n_c_rows, n_c, codes_r, n_r_rows, n_r, timbre, B, T)) {
+        h->err = "fac_dequantize: bad arguments (1 <= n_c <= rows of codes_c <= 2, n_r <= rows of codes_r <= 3, B, T > 0)";
+        return FAC_ERR_INVALID;
+    }
+    return two_pass(h, (cudaStream_t)stream, [&](Ctx& c) {
+        float* zp_cl = zp ? c.alloc<float>((size_t)B * T * LATENT) : nullptr;
+        float* zc_cl = zc ? c.alloc<float>((size_t)B * T * LATENT) : nullptr;
+        float* zr_cl = zr ? c.alloc<float>((size_t)B * T * LATENT) : nullptr;
+        float* ocl = dequantize_forward(c, codes_p, codes_c, n_c_rows, n_c, codes_r, n_r_rows, n_r, timbre, B, T, zp_cl, zc_cl, zr_cl);
+        if (c.dry) return;
+        c.check(launch_transpose(ocl, outs, B, T, LATENT, c.st), "dq.outs_T");
+        if (zp) c.check(launch_transpose(zp_cl, zp, B, T, LATENT, c.st), "dq.zp_T");
+        if (zc) c.check(launch_transpose(zc_cl, zc, B, T, LATENT, c.st), "dq.zc_T");
+        if (zr) c.check(launch_transpose(zr_cl, zr, B, T, LATENT, c.st), "dq.zr_T");
+    });
+}
+
+int fac_decode_codes(fac_handle* h, const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, int n_c, const int64_t* codes_r,
+                     int n_r_rows, int n_r, const float* timbre, int B, int T, float* y, void* stream) {
+    int rc = check_ready(h, FAC_QUANTIZER);
+    if (!rc) rc = check_ready(h, FAC_DECODER);
+    if (rc) return rc;
+    if (!y || !dequant_args_ok(codes_p, codes_c, n_c_rows, n_c, codes_r, n_r_rows, n_r, timbre, B, T)) {
+        h->err = "fac_decode_codes: bad arguments (1 <= n_c <= rows of codes_c <= 2, n_r <= rows of codes_r <= 3, B, T > 0)";
+        return FAC_ERR_INVALID;
+    }
+    return two_pass(h, (cudaStream_t)stream, [&](Ctx& c) {
+        float* ocl = dequantize_forward(c, codes_p, codes_c, n_c_rows, n_c, codes_r, n_r_rows, n_r, timbre, B, T, nullptr, nullptr,
+                                        nullptr);
+        decoder_forward(c, h->dec, ocl, B, T, y);
     });
 }
 

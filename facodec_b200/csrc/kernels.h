@@ -152,6 +152,20 @@ struct FaqParams {
     int B = 0, Tq = 0, Tz = 0, Tf0 = 0;   // Tz / Tf0 = frames per utterance of z / f0 (>= Tq)
 };
 cudaError_t launch_fa_quantize(const FaqParams& p, cudaStream_t st);
+// codes -> outs (ResidualVectorQuantize.from_codes per group + the forward_v2 AdaLN tail); indices outside [0, 1024) are
+// never dereferenced and make every channel of that frame's outs NaN
+struct DequantParams {
+    const int64_t* codes_p = nullptr;   // [B][1][T]
+    const int64_t* codes_c = nullptr;   // [B][n_c_rows][T]; rows 0 .. n_c - 1 are used
+    const int64_t* codes_r = nullptr;   // [B][n_r_rows][T]; rows 0 .. n_r - 1 are used (null when n_r = 0)
+    int n_c_rows = 0, n_c = 1, n_r_rows = 0, n_r = 0;
+    VqWeights vq[6];                    // prosody, content0, content1, residual0..2
+    const float* gamma_beta = nullptr;  // [B][2048] timbre_linear(timbre)
+    float* outs = nullptr;              // [B][T][1024]
+    float* zp = nullptr, *zc = nullptr, *zr = nullptr;  // [B][T][1024] each (may be null)
+    int B = 0, T = 0;
+};
+cudaError_t launch_dequantize(const DequantParams& p, cudaStream_t st);
 // losses[0] = commitment, losses[1] = codebook (identical in forward), from sqerr
 cudaError_t launch_vq_loss_reduce(const float* sqerr, int nq, int B, int Tq, float* losses2, cudaStream_t st);
 

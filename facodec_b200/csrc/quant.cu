@@ -31,6 +31,52 @@ __device__ __forceinline__ void store_frame(float* __restrict__ p, const float (
         *reinterpret_cast<float4*>(p + i * 128 + lane * 4) = make_float4(v[i * 4], v[i * 4 + 1], v[i * 4 + 2], v[i * 4 + 3]);
 }
 
+// out_proj (8 -> 1024) of F frames at once, channel chunk i (c = i*128 + lane*4 + 0..3):
+// o[f] = b_out + sum_k w_out[k] * zq[f][k], fmaf in k order; each w_out slice is loaded once for all F frames.
+template <int F>
+__device__ __forceinline__ void out_proj_chunk(const VqWeights& W, const float (&zq)[F][VQ_CD], int i, int lane,
+                                               float4 (&o)[F]) {
+    const float4 bo = __ldg(reinterpret_cast<const float4*>(W.b_out + i * 128 + lane * 4));
+#pragma unroll
+    for (int f = 0; f < F; ++f) o[f] = bo;
+#pragma unroll
+    for (int k = 0; k < VQ_CD; ++k) {
+        const float4 w = __ldg(reinterpret_cast<const float4*>(W.w_out + k * VQ_D + i * 128 + lane * 4));
+#pragma unroll
+        for (int f = 0; f < F; ++f) {
+            o[f].x = fmaf(w.x, zq[f][k], o[f].x);
+            o[f].y = fmaf(w.y, zq[f][k], o[f].y);
+            o[f].z = fmaf(w.z, zq[f][k], o[f].z);
+            o[f].w = fmaf(w.w, zq[f][k], o[f].w);
+        }
+    }
+}
+
+// FAquantizer.forward_v2 tail on one frame (modules/quantize.py:445-449), in place: timbre_norm = LayerNorm(1024, no
+// affine, eps 1e-5), then * gamma + beta with gb = [gamma[1024] | beta[1024]] of the frame's utterance.
+__device__ __forceinline__ void ada_ln(float (&v)[32], const float* __restrict__ gb, int lane) {
+    float s = 0.f;
+#pragma unroll
+    for (int i = 0; i < 32; ++i) s += v[i];
+    float mean = warp_sum(s) * (1.0f / VQ_D);
+    float var = 0.f;
+#pragma unroll
+    for (int i = 0; i < 32; ++i) {
+        float d = v[i] - mean;
+        var = fmaf(d, d, var);
+    }
+    float rstd = rsqrtf(warp_sum(var) * (1.0f / VQ_D) + 1e-5f);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        float4 g = __ldg(reinterpret_cast<const float4*>(gb + i * 128 + lane * 4));
+        float4 be = __ldg(reinterpret_cast<const float4*>(gb + VQ_D + i * 128 + lane * 4));
+        v[i * 4 + 0] = (v[i * 4 + 0] - mean) * rstd * g.x + be.x;
+        v[i * 4 + 1] = (v[i * 4 + 1] - mean) * rstd * g.y + be.y;
+        v[i * 4 + 2] = (v[i * 4 + 2] - mean) * rstd * g.z + be.z;
+        v[i * 4 + 3] = (v[i * 4 + 3] - mean) * rstd * g.w + be.w;
+    }
+}
+
 // One VectorQuantize.forward on the frame held in r (channel c = i*128 + lane*4 + j <-> r[i*4+j]).
 // Writes out[] = out_proj(z_q), returns the code index; sqerr = sum_k (z_e - z_q)^2.
 __device__ __forceinline__ int vq_stage(const VqWeights& W, const float (&r)[32], float (&out)[32], float& sqerr,
@@ -89,27 +135,20 @@ __device__ __forceinline__ int vq_stage(const VqWeights& W, const float (&r)[32]
     }
     float4 q0 = __ldg(reinterpret_cast<const float4*>(W.cb + bidx * VQ_CD));
     float4 q1 = __ldg(reinterpret_cast<const float4*>(W.cb + bidx * VQ_CD + 4));
-    float zq[VQ_CD] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w};
+    float zq[1][VQ_CD] = {{q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w}};
     float se = 0.f;
 #pragma unroll
     for (int k = 0; k < VQ_CD; ++k) {
-        float df = ze[k] - zq[k];
+        float df = ze[k] - zq[0][k];
         se = fmaf(df, df, se);
-        zq[k] = ze[k] + (zq[k] - ze[k]);   // straight-through estimator, forward value
+        zq[0][k] = ze[k] + (zq[0][k] - ze[k]);   // straight-through estimator, forward value
     }
     sqerr = se;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-        float4 o = __ldg(reinterpret_cast<const float4*>(W.b_out + i * 128 + lane * 4));
-#pragma unroll
-        for (int k = 0; k < VQ_CD; ++k) {
-            float4 w = __ldg(reinterpret_cast<const float4*>(W.w_out + k * VQ_D + i * 128 + lane * 4));
-            o.x = fmaf(w.x, zq[k], o.x);
-            o.y = fmaf(w.y, zq[k], o.y);
-            o.z = fmaf(w.z, zq[k], o.z);
-            o.w = fmaf(w.w, zq[k], o.w);
-        }
-        out[i * 4] = o.x; out[i * 4 + 1] = o.y; out[i * 4 + 2] = o.z; out[i * 4 + 3] = o.w;
+        float4 o[1];
+        out_proj_chunk<1>(W, zq, i, lane, o);
+        out[i * 4] = o[0].x; out[i * 4 + 1] = o[0].y; out[i * 4 + 2] = o[0].z; out[i * 4 + 3] = o[0].w;
     }
     return bidx;
 }
@@ -181,30 +220,9 @@ __global__ void __launch_bounds__(128) fa_quantize_kernel(FaqParams p) {
     }
     if (p.zr) store_frame(p.zr + fo, zr, lane);
     // outs = z_p + z_c + z_r ; timbre_norm = LayerNorm(1024, no affine), eps 1e-5 ; * gamma + beta
-    float s = 0.f;
 #pragma unroll
-    for (int i = 0; i < 32; ++i) {
-        out[i] = (zp[i] + zc[i]) + zr[i];
-        s += out[i];
-    }
-    float mean = warp_sum(s) * (1.0f / VQ_D);
-    float v = 0.f;
-#pragma unroll
-    for (int i = 0; i < 32; ++i) {
-        float d = out[i] - mean;
-        v = fmaf(d, d, v);
-    }
-    float rstd = rsqrtf(warp_sum(v) * (1.0f / VQ_D) + 1e-5f);
-    const float* gb = p.gamma_beta + (size_t)b * 2 * VQ_D;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        float4 g = __ldg(reinterpret_cast<const float4*>(gb + i * 128 + lane * 4));
-        float4 be = __ldg(reinterpret_cast<const float4*>(gb + VQ_D + i * 128 + lane * 4));
-        out[i * 4 + 0] = (out[i * 4 + 0] - mean) * rstd * g.x + be.x;
-        out[i * 4 + 1] = (out[i * 4 + 1] - mean) * rstd * g.y + be.y;
-        out[i * 4 + 2] = (out[i * 4 + 2] - mean) * rstd * g.z + be.z;
-        out[i * 4 + 3] = (out[i * 4 + 3] - mean) * rstd * g.w + be.w;
-    }
+    for (int i = 0; i < 32; ++i) out[i] = (zp[i] + zc[i]) + zr[i];
+    ada_ln(out, p.gamma_beta + (size_t)b * 2 * VQ_D, lane);
     store_frame(p.outs + fo, out, lane);
 }
 
@@ -212,6 +230,122 @@ cudaError_t launch_fa_quantize(const FaqParams& p, cudaStream_t st) {
     int nframes = p.B * p.Tq;
     if (nframes <= 0) return cudaSuccess;
     fa_quantize_kernel<<<(nframes + 3) / 4, 128, 0, st>>>(p);
+    return cudaGetLastError();
+}
+
+// Decoding from codes: ResidualVectorQuantize.from_codes (dac/nn/quantize.py:200-220) of the prosody, content and
+// residual quantizers, then the forward_v2 tail (modules/quantize.py:435-449).  Per group z_g = 0 + sum_q (W_out_q
+// cb_q[idx_q] + b_out_q) in codebook order, on the RAW codebook row (there is no z_e to straight-through against);
+// outs = (z_p + z_c) + z_r with z_r = 0 when n_r = 0; then ada_ln as fa_quantize_kernel.  One warp owns DQ_F consecutive
+// frames (lane/channel map of fa_quantize_kernel), so each w_out slice is read once per DQ_F frames (the rvq_kernel
+// lesson).  The work is chunked by channel slice i: the three group sums of one slice only need four registers per frame,
+// and the codebook rows (32 bytes, the same address for the whole warp) are re-read per slice from L1.  DQ_F = 2: the
+// 32-channel outs of four frames in registers need more than 255 registers and spill (ptxas -v); two use 226, no spills.
+// An index outside [0, 1024) is never used as an address: it reads as NaN, and every channel of that frame's outs is NaN.
+constexpr int DQ_F = 2;
+__global__ void __launch_bounds__(128) dequantize_kernel(DequantParams p) {
+    const int lane = threadIdx.x & 31;
+    const size_t nframes = (size_t)p.B * p.T;
+    const size_t f0 = ((size_t)blockIdx.x * 4 + (threadIdx.x >> 5)) * DQ_F;
+    if (f0 >= nframes) return;
+    size_t fr[DQ_F];
+    int bu[DQ_F];
+    int idx[DQ_F][6];      // codebook row per VQ (prosody, content0, content1, residual0..2); -1 = out of range
+    bool bad[DQ_F];
+#pragma unroll
+    for (int f = 0; f < DQ_F; ++f) {
+        fr[f] = f0 + f < nframes ? f0 + f : nframes - 1;   // tail: duplicate the last frame, store only valid ones
+        const int b = (int)(fr[f] / p.T), t = (int)(fr[f] - (size_t)b * p.T);
+        bu[f] = b;
+        long long raw[6];
+        raw[0] = p.codes_p[(size_t)b * p.T + t];
+#pragma unroll
+        for (int q = 0; q < 2; ++q) raw[1 + q] = q < p.n_c ? p.codes_c[((size_t)b * p.n_c_rows + q) * p.T + t] : 0;
+#pragma unroll
+        for (int q = 0; q < 3; ++q) raw[3 + q] = q < p.n_r ? p.codes_r[((size_t)b * p.n_r_rows + q) * p.T + t] : 0;
+        bad[f] = false;
+#pragma unroll
+        for (int q = 0; q < 6; ++q) {
+            const bool ok = raw[q] >= 0 && raw[q] < VQ_N;
+            idx[f][q] = ok ? (int)raw[q] : -1;
+            bad[f] |= !ok;
+        }
+    }
+    // one group's slice i: g[f] = 0 + sum over the group's first nq VQs (compile-time indices q0 .. q0 + 2)
+    auto group = [&](int q0, int nq, int i, float4 (&g)[DQ_F]) {
+#pragma unroll
+        for (int f = 0; f < DQ_F; ++f) g[f] = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+        for (int q = q0; q < q0 + 3 && q < 6; ++q) {
+            if (q - q0 >= nq) break;
+            const VqWeights& W = p.vq[q];
+            float zq[DQ_F][VQ_CD];
+#pragma unroll
+            for (int f = 0; f < DQ_F; ++f) {
+                const int j = idx[f][q];
+                float4 c0 = make_float4(__int_as_float(0x7fffffff), __int_as_float(0x7fffffff), __int_as_float(0x7fffffff),
+                                        __int_as_float(0x7fffffff));
+                float4 c1 = c0;
+                if (j >= 0) {
+                    c0 = __ldg(reinterpret_cast<const float4*>(W.cb + j * VQ_CD));
+                    c1 = __ldg(reinterpret_cast<const float4*>(W.cb + j * VQ_CD + 4));
+                }
+                zq[f][0] = c0.x; zq[f][1] = c0.y; zq[f][2] = c0.z; zq[f][3] = c0.w;
+                zq[f][4] = c1.x; zq[f][5] = c1.y; zq[f][6] = c1.z; zq[f][7] = c1.w;
+            }
+            float4 o[DQ_F];
+            out_proj_chunk<DQ_F>(W, zq, i, lane, o);
+#pragma unroll
+            for (int f = 0; f < DQ_F; ++f) {
+                g[f].x += o[f].x; g[f].y += o[f].y; g[f].z += o[f].z; g[f].w += o[f].w;
+            }
+        }
+    };
+    auto store4 = [&](float* base, int f, int i, const float4& v) {
+        if (base && f0 + f < nframes) *reinterpret_cast<float4*>(base + fr[f] * VQ_D + i * 128 + lane * 4) = v;
+    };
+    float outs[DQ_F][32];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        float4 g[DQ_F];
+        group(0, 1, i, g);                              // z_p
+#pragma unroll
+        for (int f = 0; f < DQ_F; ++f) {
+            outs[f][i * 4] = g[f].x; outs[f][i * 4 + 1] = g[f].y; outs[f][i * 4 + 2] = g[f].z; outs[f][i * 4 + 3] = g[f].w;
+            store4(p.zp, f, i, g[f]);
+        }
+        group(1, p.n_c, i, g);                          // z_c
+#pragma unroll
+        for (int f = 0; f < DQ_F; ++f) {
+            outs[f][i * 4] += g[f].x; outs[f][i * 4 + 1] += g[f].y; outs[f][i * 4 + 2] += g[f].z; outs[f][i * 4 + 3] += g[f].w;
+            store4(p.zc, f, i, g[f]);
+        }
+        group(3, p.n_r, i, g);                          // z_r (zeros when n_r = 0)
+#pragma unroll
+        for (int f = 0; f < DQ_F; ++f) {
+            outs[f][i * 4] += g[f].x; outs[f][i * 4 + 1] += g[f].y; outs[f][i * 4 + 2] += g[f].z; outs[f][i * 4 + 3] += g[f].w;
+            store4(p.zr, f, i, g[f]);
+        }
+    }
+#pragma unroll
+    for (int f = 0; f < DQ_F; ++f) {
+        ada_ln(outs[f], p.gamma_beta + (size_t)bu[f] * 2 * VQ_D, lane);
+        if (bad[f]) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i) outs[f][i] = __int_as_float(0x7fffffff);
+        }
+        if (f0 + f < nframes) store_frame(p.outs + fr[f] * VQ_D, outs[f], lane);
+    }
+}
+
+cudaError_t launch_dequantize(const DequantParams& p, cudaStream_t st) {
+    const size_t nframes = (size_t)p.B * p.T;
+    if (nframes == 0) return cudaSuccess;
+    if (p.n_c < 1 || p.n_c > 2 || p.n_r < 0 || p.n_r > 3) return cudaErrorInvalidValue;
+    const size_t per_cta = 4 * DQ_F;
+    const size_t nblk = (nframes + per_cta - 1) / per_cta;
+    if (nblk > 0x7fffffffULL) return cudaErrorInvalidValue;
+    dequantize_kernel<<<(unsigned)nblk, 128, 0, st>>>(p);
     return cudaGetLastError();
 }
 

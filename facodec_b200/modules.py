@@ -170,6 +170,56 @@ def _f32c(t):
     return t.detach().to(torch.float32).contiguous()
 
 
+CODEBOOK_SIZE = 1024
+
+
+def _codes_args(codes, timbre, n_c=None, n_r=None):
+    """Checks a ``[codes_p [B,1,T'], codes_c [B,1|2,T'], codes_r [B,0..3,T'] or None]`` list and ``timbre [B,1024]`` before
+    anything reaches the library; ``n_c`` / ``n_r`` (leading codebooks used) default to the rows given.  Returns
+    (codes_p, codes_c, codes_r or None, n_c, n_r, timbre) as contiguous int64 / float32 tensors on their own device."""
+    if len(codes) != 3:
+        raise ValueError("codes must be [codes_p, codes_c, codes_r]")
+    cp, cc, cr = codes
+    for name, t in (("codes_p", cp), ("codes_c", cc), ("codes_r", cr)):
+        if t is None and name == "codes_r":
+            continue
+        if not torch.is_tensor(t) or t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+            raise TypeError("%s must be an integer tensor" % name)
+        if t.dim() != 3:
+            raise ValueError("%s must be [B, rows, T'], got %s" % (name, tuple(t.shape)))
+    B, T = cp.shape[0], cp.shape[2]
+    rows_r = 0 if cr is None else cr.shape[1]
+    if cp.shape[1] != 1 or not (1 <= cc.shape[1] <= 2) or rows_r > 3:
+        raise ValueError("codes need 1 prosody, 1-2 content and 0-3 residual rows; got %d, %d, %d"
+                         % (cp.shape[1], cc.shape[1], rows_r))
+    for name, t in (("codes_c", cc), ("codes_r", cr)):
+        if t is not None and (t.shape[0] != B or t.shape[2] != T):
+            raise ValueError("%s is %s but codes_p is %s: B and T' must agree" % (name, tuple(t.shape), tuple(cp.shape)))
+    if B == 0 or T == 0:
+        raise ValueError("empty codes %s" % (tuple(cp.shape),))
+    n_c = cc.shape[1] if n_c is None else int(n_c)
+    n_r = rows_r if n_r is None else int(n_r)
+    if not (1 <= n_c <= cc.shape[1]) or not (0 <= n_r <= rows_r):
+        raise ValueError("need 1 <= n_c <= %d content rows and 0 <= n_r <= %d residual rows; got n_c=%d, n_r=%d"
+                         % (cc.shape[1], rows_r, n_c, n_r))
+    if not torch.is_tensor(timbre) or tuple(timbre.shape) != (B, 1024):
+        raise ValueError("timbre must be [%d, 1024], got %s" % (B, tuple(timbre.shape) if torch.is_tensor(timbre) else type(timbre)))
+    for t in (cc, cr, timbre):
+        if t is not None and t.device != cp.device:
+            raise _lib.FacError("codes and timbre must be on one device (no cross-device copies); got %s and %s"
+                                % (cp.device, t.device))
+    used = [cp, cc[:, :n_c]] + ([cr[:, :n_r]] if n_r else [])
+    bad = None
+    for t in used:
+        b = ((t < 0) | (t >= CODEBOOK_SIZE)).any()
+        bad = b if bad is None else bad | b
+    if bool(bad):
+        raise IndexError("codes out of range: every code must be in [0, %d)" % CODEBOOK_SIZE)
+    cp, cc = (t.detach().to(torch.int64).contiguous() for t in (cp, cc))
+    cr = None if cr is None else cr.detach().to(torch.int64).contiguous()
+    return cp, cc, cr, n_c, n_r, _f32c(timbre)
+
+
 class Encoder(_RefKeyModule):
     """dac/model/dac.py:69-104 Encoder(d_model=64, strides=[2,5,5,6], d_latent=1024, causal=True, lstm=2)."""
     _module_id = MOD_ENCODER
@@ -296,6 +346,30 @@ class FAquantizer(_RefKeyModule):
 
     forward_v2 = forward
 
+    def from_codes(self, codes, timbre, n_c=None, n_r=None):
+        """Codes back to the decoder's input: ResidualVectorQuantize.from_codes (dac/nn/quantize.py:200-220) of the
+        prosody, content and residual quantizers, then the forward_v2 tail (modules/quantize.py:435-449),
+        LayerNorm(z_p + z_c + z_r) * gamma + beta with (gamma, beta) = timbre_linear(timbre).
+
+        ``codes`` is the ``[codes_p, codes_c, codes_r]`` list ``forward(..., return_codes=True)`` returns and ``timbre``
+        [B, 1024] its timbre (or another utterance's: timbre conversion).  ``n_c`` / ``n_r`` use only the leading content /
+        residual codebooks (a lower bitrate; ``n_r = 0`` leaves z_r = 0); they default to the rows given.  Returns
+        ``(outs, [z_p, z_c, z_r])``, each [B, 1024, T'].  Not named ``decode``: the reference's ``decode`` takes another
+        code layout and cannot run under configs/config.yml."""
+        return self._dequantize(codes, timbre, n_c, n_r, parts=True)
+
+    def _dequantize(self, codes, timbre, n_c, n_r, parts):
+        cp, cc, cr, n_c, n_r, tv = _codes_args(codes, timbre, n_c, n_r)
+        L, h = self._prep(cp, cc, cr, tv)
+        B, _, T = cp.shape
+        dev = cp.device
+        outs = torch.empty(B, 1024, T, device=dev)
+        zp, zc, zr = (torch.empty(B, 1024, T, device=dev) for _ in range(3)) if parts else (None, None, None)
+        rc = L.fac_dequantize(h, _ptr(cp), _ptr(cc), cc.shape[1], n_c, _ptr(cr), 0 if cr is None else cr.shape[1], n_r,
+                              _ptr(tv), B, T, _ptr(outs), _ptr(zp), _ptr(zc), _ptr(zr), _stream(dev))
+        _lib.check(h, rc, "fac_dequantize")
+        return outs, [zp, zc, zr]
+
 
 class Munch(dict):
     """Attribute dict (the reference returns munch.Munch from build_model)."""
@@ -329,6 +403,21 @@ class Codec:
         rc = e.L.fac_codec_forward(e.handle, _ptr(x), B, T, n_c, _ptr(y), _ptr(cp), _ptr(cc), _ptr(cr), _ptr(timbre), _stream(dev))
         _lib.check(e.handle, rc, "fac_codec_forward")
         return y, [cp, cc, cr], timbre
+
+    def decode_codes(self, codes, timbre, n_c=None, n_r=None):
+        """Codes + timbre -> audio in one C call: model.decoder(model.quantizer.from_codes(codes, timbre, n_c, n_r)[0])
+        with the latents kept on the device.  codes = [codes_p, codes_c, codes_r] as ``forward`` returns them,
+        timbre [B, 1024] -> y [B, 1, 300 T']."""
+        if self.model.decoder.training:
+            raise NotImplementedError("eval mode only")
+        cp, cc, cr, n_c, n_r, tv = _codes_args(codes, timbre, n_c, n_r)
+        L, h = self.model.quantizer._prep(cp, cc, cr, tv)
+        B, _, T = cp.shape
+        y = torch.empty(B, 1, T * 300, device=cp.device)
+        rc = L.fac_decode_codes(h, _ptr(cp), _ptr(cc), cc.shape[1], n_c, _ptr(cr), 0 if cr is None else cr.shape[1], n_r,
+                                _ptr(tv), B, T, _ptr(y), _stream(cp.device))
+        _lib.check(h, rc, "fac_decode_codes")
+        return y
 
     def forward_host(self, x_host, n_c=2, out=None):
         """End-to-end with HOST tensors (pinned recommended): H2D, forward, D2H inside the call.
@@ -421,6 +510,14 @@ class CodecStream:
         e = self.engine
         _lib.check(e.handle, e.L.fac_stream_decode(e.handle, self.sid, _ptr(z), Fc, _ptr(y), _stream(z.device)), "fac_stream_decode")
         return y
+
+    def decode_codes(self, codes_chunk, timbre):
+        """A chunk of codes ([codes_p, codes_c, codes_r], Fc frames; the first chunk >= 10 frames) and the utterance's
+        timbre [B, 1024] -> y chunk [B, 1, 300 Fc].  Dequantizing is per frame, so the chunks together give exactly what
+        one offline ``Codec.decode_codes`` call gives."""
+        self._check(codes_chunk[0])
+        z, _ = self.model.quantizer._dequantize(codes_chunk, timbre, None, None, parts=False)
+        return self.decode(z)
 
     def close(self):
         if self.sid is not None and self.engine.handle is not None:

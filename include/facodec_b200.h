@@ -103,6 +103,25 @@ int fac_redecoder_decode(fac_handle* h, const float* z, int B, int Tf, float* y,
 int fac_voice_convert(fac_handle* h, const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, const float* timbre,
                       int B, int T, int use_p_code, int use_c_code, int n_c, float* y, void* stream);
 
+/* Decoding from codes: the codes and timbre a forward returned (or a .dac file holds, plus a timbre) back to latents /
+ * audio.  Per group (prosody, content, residual) this is ResidualVectorQuantize.from_codes (dac/nn/quantize.py:200-220):
+ * z_g = 0 + sum_q out_proj_q(codebook_q[codes[:, q]]) on the raw codebook rows; then the FAquantizer.forward_v2 tail
+ * (modules/quantize.py:435-449): outs = LayerNorm(z_p + z_c + z_r, no affine, eps 1e-5) * gamma + beta with
+ * (gamma, beta) = timbre_linear(timbre).  (The reference's own FAquantizer.decode, modules/quantize.py:244-254, expects
+ * the layout without timbre_norm and cannot run under configs/config.yml.)
+ * codes_p [B,1,T], codes_c [B,n_c_rows,T], codes_r [B,n_r_rows,T] int64 (device); the first 1 <= n_c <= n_c_rows <= 2
+ * content and 0 <= n_r <= n_r_rows <= 3 residual codebooks are used (fewer = a lower bitrate; codes_r may be NULL when
+ * n_r = 0, and then z_r = 0); timbre [B,1024].  A code outside [0, 1024) is never dereferenced: every channel of that
+ * frame's outs is NaN.  Needs the quantizer weights only.
+ * fac_dequantize: outs [B,1024,T] and (each may be NULL) zp, zc, zr [B,1024,T].
+ * fac_decode_codes: the same, then model.decoder (dac/model/dac.py:164-165) with the latents kept channels-last on the
+ * device: y [B,1,300*T].  Needs the quantizer and decoder weights. */
+int fac_dequantize(fac_handle* h, const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, int n_c, const int64_t* codes_r,
+                   int n_r_rows, int n_r, const float* timbre, int B, int T, float* outs, float* zp, float* zc, float* zr,
+                   void* stream);
+int fac_decode_codes(fac_handle* h, const int64_t* codes_p, const int64_t* codes_c, int n_c_rows, int n_c, const int64_t* codes_r,
+                     int n_r_rows, int n_r, const float* timbre, int B, int T, float* y, void* stream);
+
 /* Streaming (SURVEY.md section 8f rank 4; README.md:105-107 "causal ... can be used for streaming"): the encoder and the codec's
  * decoder are causal, so a long utterance can be processed in chunks with the SAME results as one offline call
  * (dac/model/dac.py:103-104, :164-165).  The reference ships no streaming driver; these entry points carry what the
